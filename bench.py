@@ -8,6 +8,8 @@ BASELINE.json north_star) on synthetic span streams of the shapes BASELINE.json 
     --workload {hotel,media,alibaba}   stream shape of the headline line (default hotel = configs[1] shape)
     --scaling {weak,strong}            weak: 8192 services per GPU; strong: ONE fixed list (--spans, default 100 M)
     --no-extra                         skip the extra_workloads legs (media-shaped, alibaba-shaped, shipped traces)
+    --dump-outputs DIR                 after the timed steps, write the arrays the last step returned (rank 0;
+                                       the reference arm's inputs scale with the host's core count)
 
 One "step" = one pass of the whole path (both iterations + GMM refit) over the service list.  The
 list is ONE global list partitioned across the ranks by span count (traceweaver_b200.shard); every
@@ -67,11 +69,70 @@ def parse():
     ap.add_argument("--cpu-sample", type=int, default=1536, help="services in the CPU-baseline sample")
     ap.add_argument("--no-extra", action="store_true")
     ap.add_argument("--seed", type=int, default=10)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path returned in its last step as DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
 
 
 def dist_env():
     return int(os.environ.get("RANK", 0)), int(os.environ.get("LOCAL_RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
+
+
+DUMP_BYTES = 63_000_000       # all files of --dump-outputs together, .npy headers included, stay under 64 MB
+
+
+def host_outputs(res):
+    """One step's result as host arrays: tensors copied out, distribution Params as their table."""
+    import torch
+    out = {}
+    for name, v in res.items():
+        v = getattr(v, "table", v)
+        out[name] = v.cpu().numpy() if isinstance(v, torch.Tensor) else np.asarray(v)
+    return out
+
+
+def topk_rows(flat, hb):
+    """topk_idx, laid out [in-span][rank][callee] with each service's own callee count
+    (include/traceweaver_b200.h), as one row of TW_K candidate indices per (in-span, callee) tuple, in
+    the tuple order of `assign`."""
+    from traceweaver_b200 import _abi
+    per = np.diff(hb.prob_tuple_off).astype(np.int64)
+    E = np.repeat(np.diff(hb.prob_ep_off).astype(np.int64), per)
+    t = np.arange(len(E), dtype=np.int64)
+    e = (t - np.repeat(np.asarray(hb.prob_tuple_off[:-1], np.int64), per)) % E
+    base = _abi.TW_K * (t - e) + e
+    flat = np.asarray(flat)
+    return np.stack([flat[base + r * E] for r in range(_abi.TW_K)], axis=1)
+
+
+def dump_outputs(directory, arrays, hb=None):
+    """Writes every array as DIR/<name>.npy in float64 (the integer outputs convert exactly).  topk_idx
+    is written as one top-K row per tuple (topk_rows; `hb` is the batch that was solved).  The top-K
+    score lists are NaN-padded past topk_cnt (include/traceweaver_b200.h); those empty slots are written
+    as 0, and any other non-finite value is an error.  An array larger than an equal share of DUMP_BYTES
+    keeps a fixed, seeded sample of its rows (whole rows), so that two builds run with the same
+    arguments can be compared file by file."""
+    arrays = dict(arrays)
+    if "topk_idx" in arrays:
+        arrays["topk_idx"] = topk_rows(arrays["topk_idx"], hb)
+    if "topk_score" in arrays:
+        s = np.array(arrays["topk_score"], np.float64)
+        s[np.arange(s.shape[1]) >= np.asarray(arrays["topk_cnt"])[:, None]] = 0.0
+        arrays["topk_score"] = s
+    os.makedirs(directory, exist_ok=True)
+    share = DUMP_BYTES // max(len(arrays), 1)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        if a.ndim and 8 * a.size > share:
+            keep = share // (8 * (a.size // len(a)))
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))]
+        a = a.astype(np.float64)
+        if not np.all(np.isfinite(a)):
+            raise ValueError(f"--dump-outputs: {name} holds non-finite values")
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 class ClockSampler:
@@ -234,8 +295,9 @@ def cpu_baseline(blocks, gpu_assign, n_services_sample, seed, gpu_assign_pass0=N
 
 
 def measure(args, blocks, hb, dev_index, steps, warmup, gather=None, rank=0, world=1, want_cpu=True,
-            clock=False, cpu_sample=None):
-    """All legs for one service list on this rank.  Returns a dict of raw measurements."""
+            clock=False, cpu_sample=None, want_outputs=False):
+    """All legs for one service list on this rank.  Returns a dict of raw measurements (and, with
+    want_outputs, the host copy of what the last timed step returned)."""
     import torch
     import torch.distributed as dist
     from traceweaver_b200 import synth
@@ -284,6 +346,7 @@ def measure(args, blocks, hb, dev_index, steps, warmup, gather=None, rank=0, wor
         sampler.finish()
     resident_ms = max_over_ranks(ev0.elapsed_time(ev1))
     launches = eng.launch_count() - l0
+    outputs = host_outputs(res) if want_outputs else None
     acc = accuracy(eng, res["assign"], truth, hb)
     unassigned = int(res["counters"][:, 1].sum().item())
     gather_ok = None
@@ -388,7 +451,7 @@ def measure(args, blocks, hb, dev_index, steps, warmup, gather=None, rank=0, wor
         cpu = cpu_baseline(blocks, gpu_assign, cpu_sample or args.cpu_sample, args.seed, assign_pass0, dev_index)
     return dict(n_spans=n_spans, resident_ms=resident_ms, launches=launches, accuracy=acc, unassigned=unassigned,
                 roofline=roofline, roofline_refit=roofline_refit, e2e=e2e, cpu=cpu, gather_ok=gather_ok,
-                clocks=sampler.summary() if sampler else None)
+                clocks=sampler.summary() if sampler else None, outputs=outputs)
 
 
 def shipped_directories(dev_index):
@@ -555,7 +618,9 @@ def run_ours(args):
     gather = shard.AssignGather(shard.spec_tuple_counts(specs), bounds, dev) if world > 1 else None
 
     m = measure(args, blocks, hb, local_rank, args.steps, args.warmup, gather=gather, rank=rank, world=world,
-                clock=True)
+                clock=True, want_outputs=rank == 0 and args.dump_outputs is not None)
+    if m["outputs"] is not None:
+        dump_outputs(args.dump_outputs, m["outputs"], hb)
 
     extra = []
     if rank == 0 and world == 1 and not args.no_extra:
@@ -637,7 +702,9 @@ def run_ours(args):
 def run_reference(args):
     """CPU arm: the reference's algorithm (oracle/ C port; the Python reference cannot travel to the
     GPU box and needs Gurobi), one pinned thread per physical core, each step = a bounded sample of
-    the workload sized for seconds of CPU work."""
+    the workload sized for seconds of CPU work.  The sample holds max(--cpu-sample, 24 x physical cores)
+    services so that every core has work: its inputs, and so its --dump-outputs files, repeat exactly on
+    the same host but differ between hosts with different core counts."""
     rank, _, world = dist_env()
     if rank != 0:
         return
@@ -655,7 +722,10 @@ def run_reference(args):
         run_oracle_pinned(hb, args.seed)
     dt = 0.0
     for _ in range(args.steps):
-        dt += run_oracle_pinned(hb, args.seed)[1]
+        res, t, _ = run_oracle_pinned(hb, args.seed)
+        dt += t
+    if args.dump_outputs is not None:
+        dump_outputs(args.dump_outputs, res, hb)
     v = n_spans * args.steps / dt
     sample = f"{hb.n_problems} services ({n_spans} spans) per step on {cores} pinned threads (one per physical core)"
     cfg = {"workload": WORKLOAD_TEXT[args.workload], "services_total": None, "in_spans_per_service": args.n_in,

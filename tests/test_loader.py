@@ -3,8 +3,8 @@
 1. Against the goldens: the hotel_reservation fixtures were minted from the reference's own loader
    (executor.py) on the shipped trace directories; `load_jaeger_dir` on the same directories must
    hand the engine the same arrays, the same invocation graph and the same ground truth.  The raw
-   traces live under /root/reference (25 MB per directory, not committed), so this part is skipped
-   where the reference is not mounted (the GPU box).
+   traces are the original project's data/ directory (25 MB per trace directory, not committed): set
+   TW_REFERENCE_DATA to it to run this part; without it this part is skipped.
 2. Self-contained: synthetic services are written out as Jaeger JSON files (one trace per request,
    server span -> client spans -> callee server spans) and read back; the loader must reproduce the
    generator's arrays, DAG and ground truth.
@@ -19,8 +19,8 @@ import pytest
 from golden_util import Golden
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF_ROOT = "/root/reference/data"
-REF_DATA = os.path.join(REF_ROOT, "hotel_reservation")
+REF_ROOT = os.environ.get("TW_REFERENCE_DATA", "")
+REF_DATA = os.path.join(REF_ROOT, "hotel_reservation") if REF_ROOT else ""
 GOLDENS = sorted(glob.glob(os.path.join(HERE, "golden", "hotel_load*__*.npz")) +
                  glob.glob(os.path.join(HERE, "golden", "media_load*__*.npz")) +
                  glob.glob(os.path.join(HERE, "golden", "node_load*__*.npz")))
@@ -69,7 +69,7 @@ def test_alibaba_layout_matches_reference_loader(path):
     assert np.array_equal(svc.truth, z["truth"])
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_DATA), reason="reference trace directories not mounted")
+@pytest.mark.skipif(not os.path.isdir(REF_DATA), reason="TW_REFERENCE_DATA (the original project's data/ directory) is not set")
 @pytest.mark.parametrize("path", GOLDENS, ids=[os.path.basename(p)[:-4] for p in GOLDENS])
 def test_loader_matches_reference_loader(path):
     g = Golden(path)
